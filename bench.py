@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- clips/s of the GAST-Net lifting forward (BASELINE.json metric) on N B200s.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--clips B]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--clips B] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 \
         --master-port P bench.py --gpus N --steps K --warmup W
 
@@ -342,7 +342,12 @@ def main():
     ap.add_argument('--cpu-clips', type=int, default=256, help='clips per CPU-baseline sample / reference-arm step')
     ap.add_argument('--no-cpu-baseline', action='store_true')
     ap.add_argument('--no-other-configs', action='store_true', help='headline (configs[1]) only')
+    ap.add_argument('--dump-outputs', metavar='DIR',
+                    help='after the timed steps, write the 3D poses of the last timed step as DIR/poses_3d.npy '
+                         '(float32, (clips, 1, 17, 3); the seeded inputs are the same in every run)')
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error('--steps must be at least 1')
 
     rank = int(os.environ.get('RANK', '0'))
     local_rank = int(os.environ.get('LOCAL_RANK', '0'))
@@ -400,6 +405,11 @@ def main():
         barrier()
         ms = e0.elapsed_time(e1)
         clocks = sampler.stop() if rank == 0 else None
+        if args.dump_outputs:                       # what the timed path returned to its caller in its last step
+            import numpy as np
+            os.makedirs(args.dump_outputs, exist_ok=True)
+            np.save(os.path.join(args.dump_outputs, 'poses_3d%s.npy' % ('_rank%d' % rank if rank else '')),
+                    y.cpu().numpy().astype(np.float32))
 
         # ---------------- end to end through the public API with host buffers ----------
         for i in range(3):
@@ -445,7 +455,7 @@ def main():
         del xs_dev
         model.__dict__.pop('_gast_handles', None)
         torch.cuda.empty_cache()
-        Ko, Wo = max(5, min(K, 20)), 3
+        Ko, Wo = K, W
         for name, cfg in OTHER.items():
             try:
                 other[name] = bench_other(name, cfg, device, rank, world, Ko, Wo, barrier, stream, reduce_max, peaks, peak_src)

@@ -202,6 +202,71 @@ def pipeline_cases():
     print('pipeline_17', {k: getattr(v, 'shape', None) for k, v in out.items()})
 
 
+def pipeline_random_cases():
+    """The reference's ChunkedGenerator and keypoint converters on random configurations (short videos, long
+    chunks, causal shifts, ragged last batch): every batch of every configuration.  The configurations and inputs
+    are re-drawn in tests/test_pipeline_oracle.py from the same RandomState(7) stream; only outputs are stored."""
+    from common.generators import ChunkedGenerator
+    from tools.mpii_coco_h36m import coco_h36m, mpii_h36m
+    import tools.mpii_coco_h36m as _kc
+    assert _kc.__file__.startswith(REF)
+    left, right = [4, 5, 6, 11, 12, 13], [1, 2, 3, 14, 15, 16]
+    out = {}
+    rs = np.random.RandomState(7)
+    for trial in range(6):
+        nseq = int(rs.randint(1, 5))
+        lens = [int(v) for v in rs.randint(1, 30, nseq)]
+        chunk = int(rs.choice([1, 3, 8]))
+        pad = int(rs.randint(0, 14))
+        shift = int(rs.choice([0, pad]))
+        augment = bool(rs.randint(0, 2))
+        bs = int(rs.choice([4, 7]))
+        p2 = [rs.standard_normal((n, 17, 2)).astype(np.float32) for n in lens]
+        p3 = [rs.standard_normal((n, 17, 3)).astype(np.float32) for n in lens]
+        cams = [rs.standard_normal(9).astype(np.float32) for _ in lens]
+        gen = ChunkedGenerator(bs, cams, p3, p2, chunk, pad=pad, causal_shift=shift, shuffle=True, random_seed=99,
+                               augment=augment, kps_left=left, kps_right=right, joints_left=left, joints_right=right)
+        out['t%d_num_batches' % trial] = np.array(gen.num_batches)
+        for bi, (cam, b3, b2) in enumerate(gen.next_epoch()):
+            out['t%d_b%d_cam' % (trial, bi)] = cam.astype(np.float32)
+            out['t%d_b%d_3d' % (trial, bi)] = b3.astype(np.float32)
+            out['t%d_b%d_2d' % (trial, bi)] = b2.astype(np.float32)
+    for T in (1, 5, 64):
+        k = rs.uniform(-500, 2000, (T, 17, 2)).astype(np.float32)
+        out['coco_h36m_T%d' % T], out['coco_h36m_T%d_valid' % T] = coco_h36m(k.copy())
+        k16 = rs.uniform(-500, 2000, (T, 16, 2)).astype(np.float32)
+        out['mpii_h36m_T%d' % T], out['mpii_h36m_T%d_valid' % T] = mpii_h36m(k16.copy())
+    np.savez_compressed(os.path.join(HERE, 'pipeline_17_random.npz'), **out)
+    print('pipeline_17_random', len(out), 'arrays')
+
+
+def shadowed_common_cases():
+    """What the reference's common/skeleton.py and common/graph_utils.py return for the calls its callers make
+    (h36m_dataset.py:236-247 joint removal, adj_mx_from_skeleton, adj_mx_from_edges dense and sparse): the drop-in
+    package shadows both modules, and tests/test_unchanged_callers.py holds it to these results."""
+    from common.skeleton import Skeleton as RS
+    from common.graph_utils import adj_mx_from_skeleton as r_adj_sk, adj_mx_from_edges as r_adj_ed
+    import common.graph_utils as _gu
+    assert _gu.__file__.startswith(REF)
+    h36m_parents = [-1, 0, 1, 2, 3, 4, 0, 6, 7, 8, 9, 0, 11, 12, 13, 14, 12, 16, 17, 18, 19, 20, 19, 22, 12, 24, 25, 26,
+                    27, 28, 27, 30]
+    jl, jr = [6, 7, 8, 9, 10, 16, 17, 18, 19, 20, 21, 22, 23], [1, 2, 3, 4, 5, 24, 25, 26, 27, 28, 29, 30, 31]
+    remove = [4, 5, 9, 10, 11, 16, 20, 21, 22, 23, 24, 28, 29, 30, 31]                # h36m_dataset.py:241
+    b = RS(list(h36m_parents), list(jl), list(jr))
+    kept = [int(v) for v in b.remove_joints(list(remove))]
+    out = {'has_children': np.asarray(b.has_children()), 'adj_skeleton': r_adj_sk(b).numpy()}
+    for J in (15, 16, 17, 19):
+        edges = [(i, q) for i, q in enumerate(synth.skeleton_parents(J)) if q >= 0]
+        out['adj_edges_dense_J%d' % J] = r_adj_ed(J, edges, sparse=False).numpy()
+        sp = r_adj_ed(J, edges)
+        assert sp.is_sparse
+        out['adj_edges_sparse_J%d' % J] = sp.to_dense().numpy()
+    meta = dict(kept=kept, parents=[int(v) for v in b.parents()], num_joints=int(b.num_joints()),
+                joints_left=[int(v) for v in b.joints_left()], joints_right=[int(v) for v in b.joints_right()],
+                children=[[int(c) for c in ch] for ch in b.children()])
+    save('shadowed_common', meta=meta, **out)
+
+
 def module_cases():
     J, C = 17, 32
     adj = adj_for(J)
@@ -420,9 +485,14 @@ if __name__ == '__main__':
         tc_cases()
     elif len(sys.argv) > 1 and sys.argv[1] == 'stream':
         stream_cases()
+    elif len(sys.argv) > 1 and sys.argv[1] == 'contract':
+        pipeline_random_cases()
+        shadowed_common_cases()
     else:
         main()
         tta_cases()
         pipeline_cases()
+        pipeline_random_cases()
+        shadowed_common_cases()
         train_cases()
         stream_cases()

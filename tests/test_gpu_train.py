@@ -57,7 +57,20 @@ def test_train_forward_and_gradients(J, fw, ch, B):
     p = {k: v.clone().requires_grad_(v.dtype.is_floating_point and 'running' not in k) for k, v in sd0.items()}
     stats = {}
     y_ref, loss_ref = _oracle_step(p, x, tgt, fw, J, stats)
-    loss_ref.backward()
+    # The reference's fp32 gradients move with the CPU thread count (the CPU kernels split their sums by thread), and
+    # where a (Leaky)ReLU input sits within rounding of zero they move discretely: at J=17/128ch the theta/phi biases
+    # of the last attention block are 1e-6 from fp64 at 8 and 16 threads but 8e-3 at 4 threads.  So the reference's
+    # noise is measured at fixed thread counts, the same on every machine, and its largest value is the bar.
+    g32s = []
+    nthreads = torch.get_num_threads()
+    try:
+        for nt in (1, 4, 8, 16):
+            torch.set_num_threads(nt)
+            q = {k: v.detach().clone().requires_grad_(v.requires_grad) for k, v in p.items()}
+            _oracle_step(q, x, tgt, fw, J, {})[1].backward()
+            g32s.append({k: v.grad.double() for k, v in q.items() if v.requires_grad})
+    finally:
+        torch.set_num_threads(nthreads)
     pd = {k: (v.detach().double().requires_grad_(v.requires_grad) if v.dtype.is_floating_point else v.clone())
           for k, v in p.items()}
     _, loss_d = _oracle_step(pd, x.double(), tgt.double(), fw, J, {})
@@ -78,11 +91,12 @@ def test_train_forward_and_gradients(J, fw, ch, B):
     assert int(sd1['init_bn.num_batches_tracked']) == 1
     # every parameter gradient.  fp32 gradients of this net are chaotic at the 1e-3..1e-2 level (a BatchNorm
     # output that lands on the other side of zero flips a ReLU and changes the gradient discretely), so the
-    # bar is the reference's OWN fp32 noise against fp64: in aggregate (all gradients concatenated, and the
-    # median per-tensor ratio) the CUDA path must be within 2x of it; per tensor, where single flips dominate,
-    # within 4x or an absolute floor.
+    # bar is the reference's OWN fp32 noise against fp64 (its largest over the fixed thread counts above): in
+    # aggregate (all gradients concatenated, and the median per-tensor ratio) the CUDA path must be within 2x of
+    # it; per tensor, where single flips dominate, within 4x or an absolute floor.
     bad = []
-    num_c = num_r = den = 0.0
+    num_c = den = 0.0
+    num_r = [0.0] * len(g32s)
     ratios = []
     for k, prm in m.named_parameters():
         assert prm.grad is not None, k
@@ -92,14 +106,16 @@ def test_train_forward_and_gradients(J, fw, ch, B):
             continue
         l2 = ((g - gd).norm() / gd.norm()).item()
         mx = ((g - gd).abs().max() / gd.abs().max()).item()
-        g32 = p[k].grad.double()                      # the reference port's own fp32 gradient
-        l2_ref = ((g32 - gd).norm() / gd.norm()).item()
-        mx_ref = ((g32 - gd).abs().max() / gd.abs().max()).item()
-        num_c += float((g - gd).norm() ** 2); num_r += float((g32 - gd).norm() ** 2); den += float(gd.norm() ** 2)
+        l2_ref = mx_ref = 0.0
+        for i, gs in enumerate(g32s):                 # the reference port's own fp32 gradients
+            l2_ref = max(l2_ref, ((gs[k] - gd).norm() / gd.norm()).item())
+            mx_ref = max(mx_ref, ((gs[k] - gd).abs().max() / gd.abs().max()).item())
+            num_r[i] += float((gs[k] - gd).norm() ** 2)
+        num_c += float((g - gd).norm() ** 2); den += float(gd.norm() ** 2)
         ratios.append(l2 / max(l2_ref, 1e-7))
         if not (l2 < max(5e-3, 4 * l2_ref) and mx < max(2e-2, 4 * mx_ref)):
             bad.append((k, round(l2, 5), round(l2_ref, 5), round(mx, 5), round(mx_ref, 5)))
-    agg_c, agg_r = (num_c / den) ** 0.5, (num_r / den) ** 0.5
+    agg_c, agg_r = (num_c / den) ** 0.5, (max(num_r) / den) ** 0.5
     med = float(np.median(ratios))
     _report('train_grad_noise.txt', ['J=%d fw=%s ch=%d B=%d: all-gradient rel. L2 error vs fp64: cuda %.3e, reference fp32 %.3e; '
                                      'median per-tensor ratio %.2f; per-tensor outliers %d' % (J, fw, ch, B, agg_c, agg_r, med, len(bad))])

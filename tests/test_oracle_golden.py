@@ -153,7 +153,6 @@ def test_tta_restatement_matches_reference_generator():
 @pytest.mark.parametrize('name', golden_names('train_'))
 def test_torch_ref_training_matches_reference_fixture(name):
     import torch
-    from oracle import gast_torch_ref as TR
     import train_fixture as TF
     g = load_golden(name)
     meta = g['meta']
@@ -166,6 +165,19 @@ def test_torch_ref_training_matches_reference_fixture(name):
          for k, v in m.state_dict().items()}
     masks = tuple(torch.from_numpy(a) for a in O.local_masks(adj_for(meta['J'])))
     opt = torch.optim.Adam([p[k] for k in meta['names']], lr=meta['lr'], amsgrad=meta['amsgrad'])
+    # the CPU kernels split their sums by thread: the port runs with the thread count the fixture was written with,
+    # whatever the machine's core count
+    nthreads = torch.get_num_threads()
+    torch.set_num_threads(meta['threads'])
+    try:
+        _torch_ref_training_steps(g, meta, nsteps, p, masks, opt)
+    finally:
+        torch.set_num_threads(nthreads)
+
+
+def _torch_ref_training_steps(g, meta, nsteps, p, masks, opt):
+    from oracle import gast_torch_ref as TR
+    import train_fixture as TF
     stats = {}
     for step in range(nsteps):
         x, tgt = TF.batch(meta, step)

@@ -92,19 +92,11 @@ def test_adam_amsgrad(G):
         assert np.abs(p - G['adam_p%d' % i]).max() < 2e-6, i
 
 
-@pytest.mark.skipif(not __import__('os').path.isdir('/root/reference/common'), reason='live reference only in the build container')
 def test_oracle_vs_live_reference_random_configs():
-    """Where the reference tree is present, drive its own ChunkedGenerator / converters on random configurations
-    (short videos, long chunks, causal shifts, ragged last batch) and compare the oracle bit for bit."""
-    import importlib.util
-
-    def load(name, path):
-        spec = importlib.util.spec_from_file_location(name, path)
-        mod = importlib.util.module_from_spec(spec)
-        spec.loader.exec_module(mod)
-        return mod
-    ref_gen = load('_ref_generators', '/root/reference/common/generators.py')
-    ref_kpt = load('_ref_kpts', '/root/reference/tools/mpii_coco_h36m.py')
+    """The reference's own ChunkedGenerator / converters on random configurations (short videos, long chunks, causal
+    shifts, ragged last batch; every batch of their output in tests/golden/pipeline_17_random.npz, written by
+    make_golden.py:pipeline_random_cases) against the oracle, bit for bit."""
+    R = load_golden('pipeline_17_random')
     rs = np.random.RandomState(7)
     for trial in range(6):
         nseq = int(rs.randint(1, 5))
@@ -117,22 +109,20 @@ def test_oracle_vs_live_reference_random_configs():
         p2 = [rs.standard_normal((n, 17, 2)).astype(np.float32) for n in lens]
         p3 = [rs.standard_normal((n, 17, 3)).astype(np.float32) for n in lens]
         cams = [rs.standard_normal(9).astype(np.float32) for _ in lens]
-        gen = ref_gen.ChunkedGenerator(bs, cams, p3, p2, chunk, pad=pad, causal_shift=shift, shuffle=True, random_seed=99,
-                                       augment=augment, kps_left=LEFT, kps_right=RIGHT, joints_left=LEFT, joints_right=RIGHT)
+        nb = int(R['t%d_num_batches' % trial])
         pairs = PO.chunk_pairs(lens, chunk, augment)
-        assert gen.num_batches == (len(pairs) + bs - 1) // bs
+        assert nb == (len(pairs) + bs - 1) // bs
         pairs = np.random.RandomState(99).permutation(pairs)
-        for bi, (cam, b3, b2) in enumerate(gen.next_epoch()):
+        for bi in range(nb):
             oc, o3, o2 = PO.chunk_batch(p2, p3, cams, pairs[bi * bs:(bi + 1) * bs], chunk, pad, shift, LEFT, RIGHT, LEFT, RIGHT)
-            assert np.array_equal(oc, cam.astype(np.float32)), (trial, bi)
-            assert np.array_equal(o3, b3.astype(np.float32)), (trial, bi)
-            assert np.array_equal(o2, b2.astype(np.float32)), (trial, bi)
+            assert np.array_equal(oc, R['t%d_b%d_cam' % (trial, bi)]), (trial, bi)
+            assert np.array_equal(o3, R['t%d_b%d_3d' % (trial, bi)]), (trial, bi)
+            assert np.array_equal(o2, R['t%d_b%d_2d' % (trial, bi)]), (trial, bi)
+        assert 't%d_b%d_2d' % (trial, nb) not in R
     for T in (1, 5, 64):
         k = rs.uniform(-500, 2000, (T, 17, 2)).astype(np.float32)
-        a, va = ref_kpt.coco_h36m(k.copy())
         b, vb = PO.coco_h36m(k)
-        assert np.array_equal(a, b) and np.array_equal(va, vb)
+        assert np.array_equal(R['coco_h36m_T%d' % T], b) and np.array_equal(R['coco_h36m_T%d_valid' % T], vb)
         k16 = rs.uniform(-500, 2000, (T, 16, 2)).astype(np.float32)
-        a, va = ref_kpt.mpii_h36m(k16.copy())
         b, vb = PO.mpii_h36m(k16)
-        assert np.array_equal(a, b) and np.array_equal(va, vb)
+        assert np.array_equal(R['mpii_h36m_T%d' % T], b) and np.array_equal(R['mpii_h36m_T%d_valid' % T], vb)

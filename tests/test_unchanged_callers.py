@@ -1,7 +1,7 @@
 """The reference's own callers, UNCHANGED, over the drop-in (BASELINE north_star: "trainval.py and reconstruction.py
-call it unchanged"; SURVEY.md §8b).  The caller files are not part of this repository: they are read from
-/root/reference (build container) or from baseline/_ref/ (tools/make_ref_callers.sh: git-ignored copy of the caller
-files only, never model/, so that the GPU box has them).  Without either the tests are skipped.
+call it unchanged"; SURVEY.md §8b).  The caller files are not part of this repository: build() copies them from an
+upstream GAST-Net checkout into the git-ignored oracle/_ref/ (oracle/ref_callers.py: the caller files only, never
+model/).  Without that copy the tests that run the callers are skipped.
 
 What runs unchanged: `reconstruction.reconstruction(args)` (reconstruction.py:173-267: json -> coco_h36m ->
 normalize_screen_coordinates -> UnchunkedGenerator + TTA -> model -> camera_to_world) on the real baseball clip
@@ -20,10 +20,7 @@ import torch
 from conftest import load_golden, REPO, PKG
 from gast_b200 import synth
 
-REF = next((p for p in (os.path.join(REPO, 'baseline', '_ref'), '/root/reference')
-            if os.path.exists(os.path.join(p, 'reconstruction.py'))), None)
-pytestmark = pytest.mark.skipif(REF is None, reason='reference caller files not available '
-                                                    '(run tools/make_ref_callers.sh in the build container)')
+REF = os.path.join(REPO, 'oracle', '_ref')
 
 LEFT, RIGHT = [4, 5, 6, 11, 12, 13], [1, 2, 3, 14, 15, 16]
 
@@ -32,6 +29,9 @@ LEFT, RIGHT = [4, 5, 6, 11, 12, 13], [1, 2, 3, 14, 15, 16]
 def callers():
     """import the reference's reconstruction.py and main.py with the drop-in package AHEAD of the reference root on
     sys.path (INTEGRATION.md §1) -- the only 'installation' step a user performs"""
+    if not os.path.exists(os.path.join(REF, 'reconstruction.py')):
+        pytest.skip('reference caller files not available (build() copies them into oracle/_ref/ from an upstream '
+                    'checkout, see oracle/ref_callers.py)')
     saved_path, saved_mods = list(sys.path), dict(sys.modules)
     for name in ('matplotlib', 'matplotlib.pyplot', 'matplotlib.animation', 'mpl_toolkits', 'mpl_toolkits.mplot3d'):
         if name not in sys.modules:                       # rendering back end absent from the image; never called here
@@ -66,35 +66,27 @@ def test_star_imports_resolve_to_the_drop_in(callers):
 
 def test_shadowed_common_modules_keep_the_reference_contract():
     """common/graph_utils.py and common/skeleton.py of the drop-in shadow the reference's for every caller: same
-    results, including adj_mx_from_edges' sparse default and Skeleton.remove_joints (h36m_dataset.py:236-247)."""
-    src = '/root/reference' if os.path.exists('/root/reference/common/graph_utils.py') else None
-    if src is None:
-        pytest.skip('needs the reference sources of the two shadowed modules (build container)')
-    import importlib.util
+    results, including adj_mx_from_edges' sparse default and Skeleton.remove_joints (h36m_dataset.py:236-247).
+    The reference's results are tests/golden/shadowed_common.npz (make_golden.py:shadowed_common_cases)."""
     import common.graph_utils as G
     import common.skeleton as S
-
-    def load(name):
-        spec = importlib.util.spec_from_file_location('ref_' + name, os.path.join(src, 'common', name + '.py'))
-        mod = importlib.util.module_from_spec(spec)
-        spec.loader.exec_module(mod)
-        return mod
-    RG, RS = load('graph_utils'), load('skeleton')
+    R = load_golden('shadowed_common')
+    b = R['meta']
     h36m_parents = [-1, 0, 1, 2, 3, 4, 0, 6, 7, 8, 9, 0, 11, 12, 13, 14, 12, 16, 17, 18, 19, 20, 19, 22, 12, 24, 25, 26,
                     27, 28, 27, 30]
     jl, jr = [6, 7, 8, 9, 10, 16, 17, 18, 19, 20, 21, 22, 23], [1, 2, 3, 4, 5, 24, 25, 26, 27, 28, 29, 30, 31]
-    a, b = S.Skeleton(list(h36m_parents), list(jl), list(jr)), RS.Skeleton(list(h36m_parents), list(jl), list(jr))
+    a = S.Skeleton(list(h36m_parents), list(jl), list(jr))
     remove = [4, 5, 9, 10, 11, 16, 20, 21, 22, 23, 24, 28, 29, 30, 31]                # h36m_dataset.py:241
-    assert list(a.remove_joints(list(remove))) == list(b.remove_joints(list(remove)))
-    assert list(a.parents()) == list(b.parents()) and a.num_joints() == b.num_joints() == 17
-    assert list(a.joints_left()) == list(b.joints_left()) and list(a.joints_right()) == list(b.joints_right())
-    assert np.array_equal(a.has_children(), b.has_children()) and [list(c) for c in a.children()] == [list(c) for c in b.children()]
-    assert torch.equal(G.adj_mx_from_skeleton(a), RG.adj_mx_from_skeleton(b))
+    assert list(a.remove_joints(list(remove))) == b['kept']
+    assert list(a.parents()) == b['parents'] and a.num_joints() == b['num_joints'] == 17
+    assert list(a.joints_left()) == b['joints_left'] and list(a.joints_right()) == b['joints_right']
+    assert np.array_equal(a.has_children(), R['has_children']) and [list(c) for c in a.children()] == b['children']
+    assert torch.equal(G.adj_mx_from_skeleton(a), torch.from_numpy(R['adj_skeleton']))
     for J in (15, 16, 17, 19):
         edges = [(i, q) for i, q in enumerate(synth.skeleton_parents(J)) if q >= 0]
-        assert torch.equal(G.adj_mx_from_edges(J, edges, sparse=False), RG.adj_mx_from_edges(J, edges, sparse=False))
-        sa, sb = G.adj_mx_from_edges(J, edges), RG.adj_mx_from_edges(J, edges)             # default: sparse
-        assert sa.is_sparse and sb.is_sparse and torch.equal(sa.to_dense(), sb.to_dense())
+        assert torch.equal(G.adj_mx_from_edges(J, edges, sparse=False), torch.from_numpy(R['adj_edges_dense_J%d' % J]))
+        sa = G.adj_mx_from_edges(J, edges)                                              # default: sparse
+        assert sa.is_sparse and torch.equal(sa.to_dense(), torch.from_numpy(R['adj_edges_sparse_J%d' % J]))
 
 
 def _reconstruction_args(tmp_path, weight='27_frame_model.bin'):
@@ -203,7 +195,7 @@ def test_dataparallel_branch_of_trainval(callers):
     visible: the per-forward replicas (broadcast parameter views, no `_parameters`) bind and run, eval output equals
     the single-device forward, and a training step routes gradients to the real parameters."""
     if torch.cuda.device_count() < 2:
-        pytest.skip('needs 2 GPUs (gpurun --gpus 2)')
+        pytest.skip('needs 2 GPUs (the DataParallel branch is taken only with more than one)')
     _, mn = callers
     from model.gast_net import SpatioTemporalModelOptimized1f
     from common.skeleton import Skeleton
