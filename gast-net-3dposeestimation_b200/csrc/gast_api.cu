@@ -929,6 +929,7 @@ static int forward_impl(gast_t* h, const float* x, float* y, int32_t B, int32_t 
 }
 
 static int prep_one_tc(gast_handle* h, cudaStream_t st, TcWeights& t, const float* W, int N, int K, int semch);
+static int make_perm(int J, int n, const int32_t* left, const int32_t* right, JointPerm* p);
 #include "stream.cuh"
 
 // ------------------------------------------------------------------------------------------

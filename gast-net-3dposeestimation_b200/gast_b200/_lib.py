@@ -20,6 +20,8 @@ SYMBOLS = ['gast_create', 'gast_destroy', 'gast_bind', 'gast_prepare', 'gast_out
            'gast_get_timings', 'gast_set_gemm_core', 'gast_debug_gemm', 'gast_bind_grads',
            'gast_train_workspace_bytes', 'gast_forward_train', 'gast_backward', 'gast_set_dropout_state', 'gast_tta_prepare', 'gast_tta_merge',
            'gast_stream_state_bytes', 'gast_stream_workspace_bytes', 'gast_stream_push',
+           'gast_stream_delay', 'gast_stream_delayed_state_bytes', 'gast_stream_delayed_workspace_bytes',
+           'gast_stream_push_delayed',
            'gast_chunk_gather', 'gast_keypoints_convert', 'gast_normalize_screen', 'gast_camera_to_world',
            'gast_mpjpe_workspace_bytes', 'gast_mpjpe', 'gast_p_mpjpe', 'gast_adam_chunk', 'gast_adam_step',
            'gast_last_error', 'gast_version']
@@ -101,6 +103,15 @@ def load():
     lib.gast_stream_push.argtypes = [vp, vp, C.c_int64, vp, vp, C.c_int32, vp, vp, C.c_size_t, vp]
     lib.gast_stream_push.restype = C.c_int
     ip = C.POINTER(C.c_int32)
+    lib.gast_stream_delay.argtypes = [vp]
+    lib.gast_stream_delay.restype = C.c_int32
+    lib.gast_stream_delayed_state_bytes.argtypes = [vp, C.c_int32, C.c_int32]
+    lib.gast_stream_delayed_state_bytes.restype = C.c_size_t
+    lib.gast_stream_delayed_workspace_bytes.argtypes = [vp, C.c_int32, C.c_int32]
+    lib.gast_stream_delayed_workspace_bytes.restype = C.c_size_t
+    lib.gast_stream_push_delayed.argtypes = [vp, vp, C.c_size_t, C.c_int64, vp, vp, C.c_int32, vp, vp, C.c_int32,
+                                             ip, ip, ip, ip, vp, C.c_size_t, vp]
+    lib.gast_stream_push_delayed.restype = C.c_int
     lib.gast_tta_prepare.argtypes = [vp, vp, C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.c_int32, ip, ip, vp]
     lib.gast_tta_prepare.restype = C.c_int
     lib.gast_tta_merge.argtypes = [vp, vp, C.c_int32, C.c_int32, C.c_int32, ip, ip, vp]

@@ -170,6 +170,32 @@ size_t gast_stream_workspace_bytes(gast_t* h, int32_t n_streams);
 int gast_stream_push(gast_t* h, void* state, int64_t step, const float* x, float* y, int32_t n_streams,
                      const int32_t* fresh, void* workspace, size_t workspace_bytes, void* stream);
 
+/* ---- delayed streams: non-causal models and test-time augmentation, O(1) per frame --------------------------
+ * A non-causal model (the accurate 27/81-frame checkpoints reconstruction.py and gen_skes.generate_skeletons run)
+ * streams with the same rings when its output comes `delay` frames late: the pose a push returns is that of the
+ * frame pushed `delay` pushes earlier.  gast_stream_delay = sum_i (pad_i - causal_shift_i): 0 for a causal model,
+ * (receptive_field - 1) / 2 otherwise (13 for 27 frames, 40 for 81); -1 on error.
+ * gast_stream_push_delayed: as gast_stream_push, for causal and non-causal MODEL handles (dilated or Optimized1f;
+ *   not the dense ablation), plus
+ *   hold (n_streams) int32 on the device, or null: non-zero = the stream's sequence is over; its row of x is ignored
+ *     and its newest frame is repeated.  `delay` such pushes after the last real frame return the last `delay` poses,
+ *     exactly the reference's edge padding on the right (UnchunkedGenerator(pad, causal_shift=0)).  fresh wins over
+ *     hold.  The left edge is the fresh fill of gast_stream_push.
+ *   n_sym > 0: test-time augmentation (UnchunkedGenerator(augment=True) + main.py:314-318) inside the stream: the
+ *     mirrored twin of every stream (feature 0 negated, kps_left[k] <-> kps_right[k]) runs as n_streams more rows of
+ *     the same rings, and y = mean(pose, un-flipped twin pose) with joints_left[k] <-> joints_right[k].  Index lists
+ *     are host arrays of n_sym entries; n_sym = 0 = no augmentation.
+ *   state_bytes: size of `state`, at least gast_stream_delayed_state_bytes(h, n_streams, n_sym > 0).
+ * Bitwise guarantees: with a causal model, no hold and no augmentation y equals gast_stream_push's; with augmentation
+ * y equals the un-augmented push of 2 n_streams streams fed the twins, followed by gast_tta_merge. */
+int32_t gast_stream_delay(gast_t* h);
+size_t gast_stream_delayed_state_bytes(gast_t* h, int32_t n_streams, int32_t augment);
+size_t gast_stream_delayed_workspace_bytes(gast_t* h, int32_t n_streams, int32_t augment);
+int gast_stream_push_delayed(gast_t* h, void* state, size_t state_bytes, int64_t step, const float* x, float* y,
+                             int32_t n_streams, const int32_t* fresh, const int32_t* hold, int32_t n_sym,
+                             const int32_t* kps_left, const int32_t* kps_right, const int32_t* joints_left,
+                             const int32_t* joints_right, void* workspace, size_t workspace_bytes, void* stream);
+
 /* ---- either side of the forward, on the device (SURVEY.md 8f N1-N3) --------------------------------
  * All pointers are device pointers unless marked (host).  Work is enqueued on `stream`.
  *
